@@ -42,7 +42,15 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned on rank 0 (the stream and the decompressed tensor) "
+                         "as DIR/<name>.npy in float32, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the outputs of --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------ helpers
@@ -117,6 +125,25 @@ def make_tensor(nbytes, dtype, device, seed):
         m = min(slab, n - i)
         out[i:i + m] = (torch.randn(m, generator=g, device=device, dtype=torch.float32) * sigma).to(dtype)
     return out
+
+
+DUMP_ELEMS = 1 << 22      # per output: 16 MiB of float32, so both outputs stay well under 64 MB
+
+
+def dump_outputs(out_dir, outputs):
+    """Each tensor of `outputs` ({name: tensor}) -> out_dir/<name>.npy as float32 (exact for every dtype the
+    bench codes).  A tensor with more than DUMP_ELEMS elements is sampled at DUMP_ELEMS positions drawn from a
+    fixed seed, in ascending order: the same positions for every tensor of the same length."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in outputs.items():
+        x = x.reshape(-1)
+        if x.numel() > DUMP_ELEMS:
+            g = torch.Generator().manual_seed(20240601)
+            idx = torch.randint(0, x.numel(), (DUMP_ELEMS,), generator=g).sort().values
+            x = x[idx.to(x.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), x.float().cpu().numpy())
 
 
 def cpu_reference_codec(num_buf=2, bits=1, bytes_mode=10, chunk=262144):
@@ -455,7 +482,8 @@ def run_ours(args, rank, local_rank, world):
         ev[2 * i + 1].record()
         d = ZipNN(input_format="torch").decompress(s)
         ev[2 * i + 2].record()
-        del s, d
+        if i + 1 < args.steps:
+            del s, d
     torch.cuda.synchronize()
     barrier()
     clk = clocks.stop() if rank == 0 else None
@@ -471,6 +499,9 @@ def run_ours(args, rank, local_rank, world):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         step_ms, tc_ms, td_ms = [float(x) for x in tt.tolist()]
     value = world * nbytes / (step_ms * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"stream": s, "decompressed": d})
+    del s, d
 
     # ---- e2e: host buffers through the public API (rank-local; reported for the whole job)
     e2e = None

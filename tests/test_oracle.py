@@ -1,16 +1,17 @@
 """The oracle (our C restatement) against the reference: committed golden streams, and the
-compiled reference itself when oracle/_ref is present.  CPU only."""
+compiled reference's answers on seeded blocks and streams (golden/reference_checks.json).  CPU only."""
 import hashlib
 
 import numpy as np
 import pytest
 
 from conftest import golden_stream, load_manifest
-from golden_inputs import make_input, raw_bytes
+from golden_inputs import huf_block_cases, load_reference_checks, make_input, raw_bytes, stream_cases
 from oracle import oracle as O
 from zipnn_b200 import ZipNN
 
 CASES = load_manifest()
+REF = load_reference_checks()
 
 
 def sha(b):
@@ -39,48 +40,17 @@ def test_port_reproduces_reference_stream(rec):
 
 
 def test_port_matches_compiled_reference_blocks():
-    if O.ref_cdll() is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    rng = np.random.default_rng(3)
-    for it in range(300):
-        size = int(rng.choice([12, 13, 64, 257, 1500, 4096, 65536, 131072, int(rng.integers(1, 131073))]))
-        kind = it % 5
-        if kind == 0:
-            x = (rng.standard_normal(size) * 0.02).astype(np.float32)
-            src = (x.view(np.uint32) >> 23).astype(np.uint8)
-        elif kind == 1:
-            src = rng.integers(0, 256, size, dtype=np.uint8)
-        elif kind == 2:
-            k = int(rng.integers(2, 256))
-            src = rng.choice(k, size, p=rng.dirichlet(np.ones(k) * rng.uniform(0.01, 1))).astype(np.uint8)
-        elif kind == 3:
-            src = np.full(size, 7, dtype=np.uint8)
-        else:
-            src = np.minimum(rng.geometric(rng.uniform(0.02, 0.9), size), 255).astype(np.uint8)
-        cap = 256 * 1024 if it % 2 else 128 * 1024
-        assert O.huf_compress(src, cap) == O.ref_huf_compress(src, cap)
+    for i, ((src, cap), want) in enumerate(zip(huf_block_cases(), REF["huf_blocks"], strict=True)):
+        assert sha(src) == want["input_sha256"], f"block {i}: input generator drifted"
+        r, out = O.huf_compress(src, cap)
+        assert (r, sha(out)) == (want["ret"], want["out_sha256"]), f"block {i}: {src.size} bytes, cap {cap}"
 
 
 def test_port_matches_compiled_reference_streams():
-    ref = O.ref_core()
-    if ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    rng = np.random.default_rng(11)
-    for it in range(40):
-        G = [1, 2, 4][it % 3]
-        bits = (it // 3) % 2
-        bm = 220 if G == 4 else 10
-        chunk = 128 * 1024 if G == 1 else int(rng.choice([256 * 1024, 65536, 4096]))
-        nelem = int(rng.choice([1, 3, 13, 4096, chunk // G + 1, int(rng.integers(1, 200000))]))
-        n = nelem * G
-        if it % 4 == 3:
-            data = rng.integers(0, 256, n, dtype=np.uint8)
-        else:
-            x = (rng.standard_normal(max(n // 2, 1) + 2) * 0.02).astype(np.float32)
-            data = np.ascontiguousarray((x.view(np.uint32) >> 16).astype(np.uint16).view(np.uint8)[:n])
-        h = bytearray(32)
-        h[0:2] = b"ZN"
-        r = bytes(ref.zipnn_core(bytes(h), bytearray(data.tobytes()), G, bits, bm, 0, chunk, 0.95, 10, 4))
+    h = bytearray(32)
+    h[0:2] = b"ZN"
+    for i, ((data, G, bits, bm, chunk), want) in enumerate(zip(stream_cases(), REF["streams"], strict=True)):
+        assert sha(data) == want["input_sha256"], f"stream {i}: input generator drifted"
         o = O.zipnn_compress(h, data, G, bits, bm, chunk, 0.95, threads=2).tobytes()
-        assert r == o
-        assert bytes(ref.combine_dtype(o[32:], G, bits, bm, chunk, n, 2)) == data.tobytes()
+        assert (len(o), sha(o)) == (want["stream_len"], want["stream_sha256"]), f"stream {i}: G={G} bits={bits} chunk={chunk} n={data.size}"
+        assert O.zipnn_decompress(np.frombuffer(o, dtype=np.uint8)[32:], G, bits, bm, chunk, data.size, threads=2).tobytes() == data.tobytes()

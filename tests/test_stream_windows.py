@@ -1,13 +1,16 @@
 """Window-by-window comparison of large streams with the oracle (tools/stream_windows.py).
 
 CPU part: the window logic itself, on oracle streams (whole stream vs the same chunks compressed
-alone; port vs the compiled reference).  GPU part: streams far larger than anything a whole-stream
-oracle run could cover in seconds -- 9 GiB bf16 (the group-0 size table passes 2^32 at chunk 32768)
+alone; port vs the compiled reference's recorded window streams).  GPU part: streams far larger
+than anything a whole-stream oracle run could cover in seconds -- 9 GiB bf16 (the group-0 size table passes 2^32 at chunk 32768)
 and 6 GiB fp32 (groups 2 and 3 start beyond 2^32) -- compared with the oracle on windows that
 include the chunks around every 2^32 crossing (u64 size table, csrc/zipnn_core.c:145-153)."""
+import hashlib
+
 import numpy as np
 import pytest
 
+from golden_inputs import WINDOW_CASE, gauss_bytes, load_reference_checks, window_case_bytes
 from oracle import oracle as O
 from tools.stream_windows import StreamTables, check_stream_windows, compare_window
 
@@ -18,19 +21,12 @@ def _hdr():
     return h
 
 
-def _gauss_bytes(rng, n, esz):
-    x = (rng.standard_normal(n // esz + 2) * 0.02).astype(np.float32)
-    if esz == 2:
-        return np.ascontiguousarray((x.view(np.uint32) >> 16).astype(np.uint16).view(np.uint8)[:n])
-    return np.ascontiguousarray(x.view(np.uint8)[:n])
-
-
 @pytest.mark.parametrize("G,bits,chunk", [(2, 1, 4096), (4, 1, 65536), (1, 0, 131072), (2, 0, 262144)])
 def test_windows_of_an_oracle_stream_match_the_chunks_compressed_alone(G, bits, chunk):
     rng = np.random.default_rng(5 + G)
     K = 37
     n = (K - 1) * chunk + (chunk // 2 // G) * G          # ragged last chunk
-    data = _gauss_bytes(rng, n, 2 if G <= 2 else 4)
+    data = gauss_bytes(rng, n, 2 if G <= 2 else 4)
     data[3 * chunk: 4 * chunk] = 0                        # an RLE chunk
     data[5 * chunk: 6 * chunk] = rng.integers(0, 256, chunk, dtype=np.uint8)   # an all-raw chunk
     bm = 220 if G == 4 else 10
@@ -51,18 +47,19 @@ def test_windows_of_an_oracle_stream_match_the_chunks_compressed_alone(G, bits, 
 
 
 def test_windows_against_the_compiled_reference():
-    ref = O.ref_core()
-    if ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    rng = np.random.default_rng(8)
-    chunk, G, K = 262144, 2, 9
-    n = K * chunk
-    data = _gauss_bytes(rng, n, 2)
+    """The reference's streams for two chunk ranges alone (recorded in golden/reference_checks.json) are
+    windows of the port's whole stream."""
+    want = load_reference_checks()
+    data = window_case_bytes()
+    assert hashlib.sha256(data.tobytes()).hexdigest() == want["window_input_sha256"], "input generator drifted"
+    chunk, G, K = WINDOW_CASE["chunk"], WINDOW_CASE["G"], WINDOW_CASE["K"]
     whole = O.zipnn_compress(_hdr(), data, G, 1, 10, chunk, 0.95, threads=4)
     tab = StreamTables(whole, 32, G, K)
-    for c0, c1 in [(0, 3), (4, 9)]:
-        r = np.frombuffer(bytes(ref.zipnn_core(bytes(_hdr()), bytearray(data[c0 * chunk: c1 * chunk].tobytes()), G, 1, 10, 0, chunk, 0.95, 10, 4)),
-                          dtype=np.uint8)
+    for (c0, c1), rec in zip(WINDOW_CASE["windows"], want["windows"], strict=True):
+        assert rec["chunks"] == [c0, c1]
+        # the port's stream for the window equals the reference's, so it can stand in for it
+        r = O.zipnn_compress(_hdr(), data[c0 * chunk: c1 * chunk], G, 1, 10, chunk, 0.95, threads=4)
+        assert (r.size, hashlib.sha256(r.tobytes()).hexdigest()) == (rec["stream_len"], rec["stream_sha256"])
         assert compare_window(tab, c0, c1, r, 32) > 0
 
 

@@ -459,8 +459,13 @@ __device__ __forceinline__ void tile_to_global(const uint8_t* tile, uint8_t* dst
   if ((uint32_t)tid < cnt - done) dst[done + tid] = tile[done + tid];
 }
 
-// Canonical code values from lengths, one warp (huf_compress.c:390-407).
-template <bool kValHigh>
+// Canonical code values from lengths, one warp (huf_compress.c:390-407).  Entry formats:
+//   kLeftAligned = false: val | nb << 16 (k_encode_write);
+//   kLeftAligned = true : val << (32 - nb) | nb, 0 for an absent symbol (k_encode_write_warp).  The value sits at
+//                         the top of the word and the length in bits 0..4 (bits 5..20 are zero), so a wrapping
+//                         funnel shift by the entry itself appends the code to a run in one instruction, and sums
+//                         of entries carry the exact sum of lengths in their low 21 bits (see wb_run).
+template <bool kLeftAligned>
 __device__ __forceinline__ void warp_build_codes(const uint8_t* nb, int lg, uint32_t* code) {
   const int lane = threadIdx.x & 31;
   uint32_t per_len[kHufLogMax + 1];
@@ -493,7 +498,7 @@ __device__ __forceinline__ void warp_build_codes(const uint8_t* nb, int lg, uint
       if (mine == l) val = start[l] + __popc(m & ((1u << lane) - 1u));
       start[l] += __popc(m);
     }
-    code[base + lane] = kValHigh ? ((val << 8) | (uint32_t)mine) : (val | ((uint32_t)mine << 16));
+    code[base + lane] = kLeftAligned ? (mine ? (val << (32 - mine)) | (uint32_t)mine : 0u) : (val | ((uint32_t)mine << 16));
   }
 }
 
@@ -669,16 +674,60 @@ __global__ void __launch_bounds__(kEncThreads) k_encode_write(const uint8_t* __r
 // (huf_compress.c:552-603) and a contiguous quarter of each raw plane.  The chunk is read
 // once (128-bit loads, the next tile prefetched), split in registers, and every plane is
 // finished by the same warp: no block-wide synchronisation after the per-chunk setup.
-//   coded plane: 16 symbols per lane -> 4 runs of <= 44 bits, warp suffix scan of the bit
-//                lengths (the last symbol is emitted first, huf_compress.c:474-499), OR into a
-//                warp-private bit buffer whose words are aligned with the destination's
-//                32-bit words, coalesced flush of the completed words;
-//   raw plane  : 512 bytes staged in shared memory, written with aligned 128-bit stores
+// A warp step covers H halves of 512 plane bytes; a lane holds 16 bytes of each half.
+//   coded plane: 16 symbols per lane and half -> 4 runs of <= 44 bits each, ONE warp suffix
+//                scan of the bit lengths of all halves (the last symbol is emitted first,
+//                huf_compress.c:474-499), OR into a warp-private bit buffer whose words are
+//                aligned with the destination's 32-bit words, coalesced flush of the completed
+//                words;
+//   raw plane  : the step's bytes staged in shared memory, written with aligned 128-bit stores
 //                (funnel-shifted to the destination's alignment), byte stores at the edges.
 // =====================================================================================
 constexpr int kWbWarps = 4;
-constexpr uint32_t kWbTile = 512;                          // plane bytes per warp step (16 per lane)
-constexpr uint32_t kWbBitWords = (kWbTile * 11) / 32 + 4;  // worst-case tile bits + carry
+
+// H = 2 (32 symbols per lane per step) pays the scan, the flush, the loop head and the raw plane's
+// edge bytes once per 1024 plane bytes.  fp32's four planes keep H = 1: its step already needs
+// about 120 registers.
+template <int G>
+struct WbCfg {
+  static constexpr int H = (G == 4) ? 1 : 2;
+  static constexpr uint32_t kTile = 512u * H;                    // plane bytes per warp step
+  // CTAs per SM the register budget has to allow: G = 1 72 registers, G = 2 96, G = 4 121 (sm_100a, no spills)
+  static constexpr int kMinBlocks = (G == 4) ? 4 : (G == 2 ? 5 : 7);
+  // worst case: 11-bit codes on every symbol, behind a carry of < 32 bits; the last run's third word
+  // lies at most two words past the word holding its first bit
+  static constexpr uint32_t kBitWords = (kTile * 11 + 31) / 32 + 3;
+};
+
+// The four symbols of plane word w, byte 3 first (emission order), as one run of <= 44 bits (lo, hi).
+// Entries are left-aligned (warp_build_codes<true>): __funnelshift_l(e, x, e) = x << n | code, so a
+// pair costs two funnel shifts and needs no field extraction.  len holds the run's bit length in its
+// low 21 bits; the bits above are garbage from the code values (every consumer masks or uses only
+// the low 5 bits through a wrapping shift).
+__device__ __forceinline__ void wb_run(const unsigned char* code, uint32_t w, uint32_t& lo, uint32_t& hi, uint32_t& len) {
+  const uint32_t e3 = *reinterpret_cast<const uint32_t*>(code + ((w >> 22) & 0x3FCu));
+  const uint32_t e2 = *reinterpret_cast<const uint32_t*>(code + ((w >> 14) & 0x3FCu));
+  const uint32_t e1 = *reinterpret_cast<const uint32_t*>(code + ((w >> 6) & 0x3FCu));
+  const uint32_t e0 = *reinterpret_cast<const uint32_t*>(code + ((w << 2) & 0x3FCu));
+  const uint32_t pa = __funnelshift_l(e3, __funnelshift_l(e2, 0u, e2), e3);  // code3 | code2 << n3
+  const uint32_t pb = __funnelshift_l(e1, __funnelshift_l(e0, 0u, e0), e1);  // code1 | code0 << n1
+  const uint32_t la = e3 + e2;                                               // n3 + n2 (2..22) in the low bits
+  lo = pa | __funnelshift_l(0u, pb, la);
+  hi = __funnelshift_l(pb, 0u, la);
+  len = la + e1 + e0;
+}
+
+// OR a run of <= 44 bits into the bit buffer at bit offset off (garbage above bit 20 allowed): three
+// unconditional reductions, the words that receive no bits get an OR of zero.
+__device__ __forceinline__ void wb_place(uint32_t bitbuf_s, uint32_t off, uint32_t lo, uint32_t hi) {
+  const uint32_t sa = bitbuf_s + ((off >> 3) & 0xFFFCu);
+  const uint32_t w0 = __funnelshift_l(0u, lo, off);  // lo << s
+  const uint32_t w1 = __funnelshift_l(lo, hi, off);  // hi << s | lo >> (32 - s); hi when s = 0
+  const uint32_t w2 = __funnelshift_l(hi, 0u, off);  // hi >> (32 - s); 0 when s = 0
+  asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(sa), "r"(w0) : "memory");
+  asm volatile("red.shared.or.b32 [%0+4], %1;" ::"r"(sa), "r"(w1) : "memory");
+  asm volatile("red.shared.or.b32 [%0+8], %1;" ::"r"(sa), "r"(w2) : "memory");
+}
 
 // (lo, hi) = 4 bytes each of the two top byte planes of 4 elements; the element-level rotation
 // [sign][exp8][mant] -> [exp8][sign][mant] (data_manipulation_dtype16.c:10-20, dtype32.c:39-49) becomes
@@ -700,12 +749,19 @@ struct WbItem {
 
 template <int G>
 struct WbSmem {
-  uint32_t code[G][256];                       // val << 8 | nb
+  uint32_t code[G][256];                       // val << (32 - nb) | nb (warp_build_codes<true>)
   WbItem item[G];
   __align__(16) uint8_t nb[G][256];
-  uint32_t bitbuf[kWbWarps][G][kWbBitWords];
-  __align__(16) uint8_t stage[kWbWarps][kWbTile + 32];
+  uint32_t bitbuf[kWbWarps][G][WbCfg<G>::kBitWords];
+  __align__(16) uint8_t stage[kWbWarps][WbCfg<G>::kTile + 32];
 };
+static_assert(WbCfg<2>::kBitWords * 4 <= 0xFFFCu, "wb_place masks the word offset to 16 bits");
+// Pass B relies on codes of at most 11 bits: the left-aligned entries keep bits 5..20 clear (so sums of
+// entries carry exact lengths in bits 0..20) and kBitWords is sized for 11 bits per symbol.  Pass A's table
+// log is fse_pick_log(kHufLogDefault, ...), which is at most max(kHufLogDefault, 9) for byte symbols (the
+// minimum log for 256 symbols is 9), and the code lengths are limited to it.  kHufLogMax (12) is only what
+// the format allows a decoder to meet.
+static_assert(kHufLogDefault <= 11, "k_encode_write_warp's entry format and bit buffer assume codes of <= 11 bits");
 
 // Per-stream bit writer state kept in registers by every lane of the warp (uniform values).
 struct WbStream {
@@ -738,7 +794,7 @@ __device__ __forceinline__ void wb_flush(uint32_t* bitbuf, WbStream& st, int lan
 }
 
 template <int G>
-__global__ void __launch_bounds__(kWbWarps * 32) k_encode_write_warp(const uint8_t* __restrict__ in, uint64_t n, uint32_t chunk,
+__global__ void __launch_bounds__(kWbWarps * 32, WbCfg<G>::kMinBlocks) k_encode_write_warp(const uint8_t* __restrict__ in, uint64_t n, uint32_t chunk,
                                                                      uint64_t K, int bits_mode, const uint8_t* __restrict__ types,
                                                                      const uint32_t* __restrict__ sizes,
                                                                      const EncSave* __restrict__ saves,
@@ -786,91 +842,116 @@ __global__ void __launch_bounds__(kWbWarps * 32) k_encode_write_warp(const uint8
     __syncthreads();
 
     // ---- warp `warp` = stream index ----
+    using Cfg = WbCfg<G>;
+    constexpr int H = Cfg::H;
+    constexpr uint32_t kTile = Cfg::kTile;
     const int s = warp;
     WbStream st[G];
     uint32_t raw_shift[G];  // destination misalignment of the raw plane quarter (bytes, mod 16)
+    uint32_t kind[G];       // what the tile loop does with plane g: 0 raw, 1 coded, 2 nothing (RLE)
 #pragma unroll
     for (int g = 0; g < G; g++) {
       const WbItem& it = S.item[g];
       st[g].gaddr = it.dest;
       st[g].a = st[g].B = st[g].flushed = 0;
       raw_shift[g] = 0;
-      if (it.type == 1 && it.size > 1) {
+      kind[g] = it.type == 0 ? 0u : (it.size > 1 ? 1u : 2u);
+      if (kind[g] == 1) {
         uint32_t at = it.hsize + 6;
         for (int q = 0; q < s; q++) at += it.sbytes[q];
         st[g].gaddr = it.dest + at;
         st[g].a = (uint32_t)((uintptr_t)st[g].gaddr & 3);
         st[g].B = 8 * st[g].a;
-        for (uint32_t w = lane; w < kWbBitWords; w += 32) S.bitbuf[warp][g][w] = 0;
-      } else if (it.type == 0) {
+        for (uint32_t w = lane; w < Cfg::kBitWords; w += 32) S.bitbuf[warp][g][w] = 0;
+      } else if (kind[g] == 0) {
         st[g].gaddr = it.dest + (uint64_t)s * seg;
         raw_shift[g] = (uint32_t)((uintptr_t)st[g].gaddr & 15);
       }
     }
     __syncwarp();
 
+    // Lane `lane` holds plane bytes [512 h + 16 lane, +16) of the tile, h < H.
     const uint8_t* src_s = in_c + (uint64_t)s * seg * G;
-    const uint32_t ntiles = (seg + kWbTile - 1) / kWbTile;
-    uint4 cur[G], nxt[G];
+    const uint32_t ntiles = (seg + kTile - 1) / kTile;
+    uint4 cur[H][G], nxt[H][G];
     {
-      const uint32_t t0 = (ntiles - 1) * kWbTile;
-      if (t0 + 16 * lane < seg) {
-        const uint4* p = reinterpret_cast<const uint4*>(src_s + (uint64_t)(t0 + 16 * lane) * G);
+      const uint32_t t0 = (ntiles - 1) * kTile;
 #pragma unroll
-        for (int i = 0; i < G; i++) nxt[i] = __ldg(p + i);
+      for (int h = 0; h < H; h++) {
+        if (t0 + 512u * h + 16 * lane < seg) {
+          const uint4* p = reinterpret_cast<const uint4*>(src_s + (uint64_t)(t0 + 512u * h + 16 * lane) * G);
+#pragma unroll
+          for (int i = 0; i < G; i++) nxt[h][i] = __ldg(p + i);
+        }
       }
     }
     // Tiles run from the end of the stream to its start (huff0 emits the last symbol first); only the
     // first one processed can be partial, so the others are compiled with `have` known to be true.
     auto do_tile = [&](auto full_tag, const uint32_t ti) {
       constexpr bool kFull = decltype(full_tag)::value;
-      const uint32_t t0 = ti * kWbTile;
-      const uint32_t cnt = kFull ? kWbTile : min(kWbTile, seg - t0);  // multiple of 16
-      const bool have = kFull ? true : (16u * lane < cnt);
+      const uint32_t t0 = ti * kTile;
+      const uint32_t cnt = kFull ? kTile : min(kTile, seg - t0);  // multiple of 16
+      bool have[H];
 #pragma unroll
-      for (int i = 0; i < G; i++) cur[i] = nxt[i];
+      for (int h = 0; h < H; h++) have[h] = kFull ? true : (512u * h + 16u * lane < cnt);
+#pragma unroll
+      for (int h = 0; h < H; h++)
+#pragma unroll
+        for (int i = 0; i < G; i++) cur[h][i] = nxt[h][i];
       if (ti > 0) {  // prefetch the next (lower) tile, always full
-        const uint4* p = reinterpret_cast<const uint4*>(src_s + (uint64_t)(t0 - kWbTile + 16 * lane) * G);
 #pragma unroll
-        for (int i = 0; i < G; i++) nxt[i] = __ldg(p + i);
-      }
-      uint4 pv[G];
-      if (have) {
-        uint32_t w[4 * G];
+        for (int h = 0; h < H; h++) {
+          const uint4* p = reinterpret_cast<const uint4*>(src_s + (uint64_t)(t0 - kTile + 512u * h + 16 * lane) * G);
 #pragma unroll
-        for (int i = 0; i < G; i++) {
-          w[4 * i] = cur[i].x; w[4 * i + 1] = cur[i].y; w[4 * i + 2] = cur[i].z; w[4 * i + 3] = cur[i].w;
+          for (int i = 0; i < G; i++) nxt[h][i] = __ldg(p + i);
         }
-        split16<G>(w, pv);
-        if (rot) {  // sign-bit rotation at plane level: 4 operations per 4 elements instead of 5 per word
-          rotate_planes(pv[(G - 2) % G].x, pv[G - 1].x);
-          rotate_planes(pv[(G - 2) % G].y, pv[G - 1].y);
-          rotate_planes(pv[(G - 2) % G].z, pv[G - 1].z);
-          rotate_planes(pv[(G - 2) % G].w, pv[G - 1].w);
+      }
+      uint4 pv[H][G];
+#pragma unroll
+      for (int h = 0; h < H; h++) {
+        if (have[h]) {
+          uint32_t w[4 * G];
+#pragma unroll
+          for (int i = 0; i < G; i++) {
+            w[4 * i] = cur[h][i].x; w[4 * i + 1] = cur[h][i].y; w[4 * i + 2] = cur[h][i].z; w[4 * i + 3] = cur[h][i].w;
+          }
+          split16<G>(w, pv[h]);
+          if (rot) {  // sign-bit rotation at plane level: 4 operations per 4 elements instead of 5 per word
+            rotate_planes(pv[h][(G - 2) % G].x, pv[h][G - 1].x);
+            rotate_planes(pv[h][(G - 2) % G].y, pv[h][G - 1].y);
+            rotate_planes(pv[h][(G - 2) % G].z, pv[h][G - 1].z);
+            rotate_planes(pv[h][(G - 2) % G].w, pv[h][G - 1].w);
+          }
         }
       }
 #pragma unroll
       for (int g = 0; g < G; g++) {
-        const uint32_t type = S.item[g].type, size = S.item[g].size;
-        if (type == 0) {
-          // ---- raw plane: 16 bytes per lane -> dest + t0 .. ----
-          uint8_t* stg = S.stage[warp];
-          if (have) *reinterpret_cast<uint4*>(stg + 16 * lane) = pv[g];
-          __syncwarp();
+        if (kind[g] == 0) {
+          // ---- raw plane: 16 bytes per lane and half -> dest + t0 .. ----
           uint8_t* D = st[g].gaddr + t0;
           const uint32_t m = raw_shift[g];
           if (m == 0) {
-            if (have) *reinterpret_cast<uint4*>(D + 16 * lane) = pv[g];
+#pragma unroll
+            for (int h = 0; h < H; h++)
+              if (have[h]) *reinterpret_cast<uint4*>(D + 512u * h + 16 * lane) = pv[h][g];
           } else {
+            uint8_t* stg = S.stage[warp];
+#pragma unroll
+            for (int h = 0; h < H; h++)
+              if (have[h]) *reinterpret_cast<uint4*>(stg + 512u * h + 16 * lane) = pv[h][g];
+            __syncwarp();
             const uint32_t head = 16 - m;  // bytes before the first aligned destination block
             const uint32_t nblk = (cnt - head) >> 4;
-            {  // every lane computes (the stage has 32 spare bytes behind the tile); only the store is conditional
-              const uint4 a4 = *reinterpret_cast<const uint4*>(stg + 16 * lane);
-              const uint4 b4 = *reinterpret_cast<const uint4*>(stg + 16 * lane + 16);
+            const uint32_t bs = (head & 3) * 8;
+#pragma unroll
+            for (int h = 0; h < H; h++) {
+              // every lane computes (the stage has 32 spare bytes behind the tile); only the store is conditional
+              const uint32_t blk = 32u * h + (uint32_t)lane;
+              const uint4 a4 = *reinterpret_cast<const uint4*>(stg + 16 * blk);
+              const uint4 b4 = *reinterpret_cast<const uint4*>(stg + 16 * blk + 16);
               const uint32_t wv[8] = {a4.x, a4.y, a4.z, a4.w, b4.x, b4.y, b4.z, b4.w};
               // 16 bytes starting `head` bytes into (a4, b4): the word part of the shift is uniform over
               // the warp, so it is a 4-way switch (4 funnel shifts) rather than 7 shifts + 9 selects
-              const uint32_t bs = (head & 3) * 8;
               uint32_t o[4];
               switch (head >> 2) {
                 case 0:
@@ -890,11 +971,11 @@ __global__ void __launch_bounds__(kWbWarps * 32) k_encode_write_warp(const uint8
                   for (int i = 0; i < 4; i++) o[i] = __funnelshift_r(wv[i + 3], wv[i + 4], bs);
                   break;
               }
-              if ((uint32_t)lane < nblk) *reinterpret_cast<uint4*>(D + head + 16 * lane) = make_uint4(o[0], o[1], o[2], o[3]);
+              if (blk < nblk) *reinterpret_cast<uint4*>(D + head + 16 * blk) = make_uint4(o[0], o[1], o[2], o[3]);
             }
-            if (kFull) {  // the 16 bytes around the 31 aligned blocks: head bytes in front, 16 - head behind
+            if (kFull) {  // the 16 bytes around the aligned blocks: head bytes in front, 16 - head behind
               if (lane < 16) {
-                const uint32_t idx = (uint32_t)lane < head ? (uint32_t)lane : (kWbTile - 16u + (uint32_t)lane);
+                const uint32_t idx = (uint32_t)lane < head ? (uint32_t)lane : (kTile - 16u + (uint32_t)lane);
                 D[idx] = stg[idx];
               }
             } else {
@@ -902,71 +983,70 @@ __global__ void __launch_bounds__(kWbWarps * 32) k_encode_write_warp(const uint8
               const uint32_t done = head + 16 * nblk;
               if ((uint32_t)lane < cnt - done) D[done + lane] = stg[done + lane];
             }
+            __syncwarp();
           }
-          __syncwarp();
-        } else if (size > 1) {
-          // ---- coded plane: this lane's 16 symbols, last byte first ----
-          // Run r = symbols 4r..4r+3 = bytes 3,2,1,0 of word 3-r.  Table entries are val << 8 | nb;
-          // the byte is turned into the table's byte offset with one shift + one mask, two codes are
-          // joined in 32 bits (<= 22), two pairs in 64 (<= 44).
+        } else if (kind[g] == 1) {
+          // ---- coded plane: this lane's 16 symbols of each half, last byte first ----
+          // Run r of half h = symbols 4r..4r+3 = bytes 3,2,1,0 of word 3-r (wb_run).  Half H-1 is
+          // emitted before half H-2, so ONE suffix scan over the lanes of the halves' lengths packed in
+          // 16-bit fields (<= 512 * 11 bits per half) places all of them.
           const unsigned char* code = reinterpret_cast<const unsigned char*>(S.code[g]);
-          uint64_t v[4] = {0, 0, 0, 0};
-          uint32_t l[4] = {0, 0, 0, 0};
-          if (have) {
-            const uint32_t wv[4] = {pv[g].x, pv[g].y, pv[g].z, pv[g].w};
+          uint32_t lo[H][4], hi[H][4], len[H][4], mine[H];
 #pragma unroll
-            for (int r = 0; r < 4; r++) {
-              const uint32_t w = wv[3 - r];
-              const uint32_t e3 = *reinterpret_cast<const uint32_t*>(code + ((w >> 22) & 0x3FCu));
-              const uint32_t e2 = *reinterpret_cast<const uint32_t*>(code + ((w >> 14) & 0x3FCu));
-              const uint32_t e1 = *reinterpret_cast<const uint32_t*>(code + ((w >> 6) & 0x3FCu));
-              const uint32_t e0 = *reinterpret_cast<const uint32_t*>(code + ((w << 2) & 0x3FCu));
-              const uint32_t n3 = e3 & 0xFFu, n2 = e2 & 0xFFu, n1 = e1 & 0xFFu, n0 = e0 & 0xFFu;
-              const uint32_t hi = (e3 >> 8) | ((e2 >> 8) << n3);  // emitted first
-              const uint32_t lo = (e1 >> 8) | ((e0 >> 8) << n1);
-              const uint32_t lh = n3 + n2;
-              v[r] = (uint64_t)hi | ((uint64_t)lo << lh);
-              l[r] = lh + n1 + n0;
+          for (int h = 0; h < H; h++) {
+            if (have[h]) {
+              const uint32_t wv[4] = {pv[h][g].x, pv[h][g].y, pv[h][g].z, pv[h][g].w};
+#pragma unroll
+              for (int r = 0; r < 4; r++) wb_run(code, wv[3 - r], lo[h][r], hi[h][r], len[h][r]);
+              mine[h] = (len[h][0] + len[h][1] + len[h][2] + len[h][3]) & 0x1FFFFFu;
+            } else {  // an idle lane of the partial tile ORs zeros at a valid offset
+#pragma unroll
+              for (int r = 0; r < 4; r++) lo[h][r] = hi[h][r] = len[h][r] = 0;
+              mine[h] = 0;
             }
           }
-          const uint32_t mine = l[0] + l[1] + l[2] + l[3];
-          uint32_t x = mine;  // suffix sum over lanes: lane 31 is emitted first
+          const uint32_t packed = (H == 2) ? (mine[H - 1] | (mine[0] << 16)) : mine[0];
+          uint32_t x = packed;  // suffix sum over lanes: lane 31 is emitted first
 #pragma unroll
           for (int o = 1; o < 32; o <<= 1) {
             const uint32_t y = __shfl_down_sync(0xffffffffu, x, o);
             if (lane + o < 32) x += y;
           }
-          const uint32_t tile_bits = __shfl_sync(0xffffffffu, x, 0);
+          const uint32_t tot = __shfl_sync(0xffffffffu, x, 0);
+          const uint32_t ex = x - packed;  // the fields never borrow: each is >= this lane's part
           uint32_t* bitbuf = S.bitbuf[warp][g];
-          uint32_t off = (st[g].B - 32 * st[g].flushed) + (x - mine);
-          // Branch-free: a run of <= 44 bits touches words wi, wi+1 (always written, OR of 0 is harmless,
-          // an idle lane of the last partial tile ORs zeros at a valid offset) and, when it starts past
-          // bit 20, wi+2 (predicated reduction, no branch around it).
           const uint32_t bitbuf_s = (uint32_t)__cvta_generic_to_shared(bitbuf);
+          const uint32_t base = st[g].B - 32 * st[g].flushed;
+          uint32_t off[H], tile_bits;
+          if constexpr (H == 2) {
+            off[H - 1] = base + (ex & 0xFFFFu);
+            off[0] = base + (tot & 0xFFFFu) + (ex >> 16);
+            tile_bits = (tot & 0xFFFFu) + (tot >> 16);
+          } else {
+            off[0] = base + ex;
+            tile_bits = tot;
+          }
 #pragma unroll
-          for (int r = 0; r < 4; r++) {
-            const uint32_t sh = off & 31, sa = bitbuf_s + ((off >> 5) << 2);
-            const uint32_t lo32 = (uint32_t)v[r], hi32 = (uint32_t)(v[r] >> 32);
-            const uint32_t w0 = lo32 << sh;
-            const uint32_t w1 = __funnelshift_l(lo32, hi32, sh);
-            const uint32_t w2 = (hi32 >> 1) >> (31 - sh);
-            asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(sa), "r"(w0) : "memory");
-            asm volatile("red.shared.or.b32 [%0+4], %1;" ::"r"(sa), "r"(w1) : "memory");
-            asm volatile("{ .reg .pred p; setp.ne.u32 p, %1, 0; @p red.shared.or.b32 [%0+8], %1; }" ::"r"(sa), "r"(w2) : "memory");
-            off += l[r];
+          for (int h = 0; h < H; h++) {
+            uint32_t o = off[h];
+#pragma unroll
+            for (int r = 0; r < 4; r++) {
+              wb_place(bitbuf_s, o, lo[h][r], hi[h][r]);
+              o += len[h][r];
+            }
           }
           __syncwarp();
           st[g].B += tile_bits;
           wb_flush(bitbuf, st[g], lane);
         }
       }
-        };
+    };
     do_tile(std::false_type{}, ntiles - 1);
     for (uint32_t ti = ntiles - 1; ti-- > 0;) do_tile(std::true_type{}, ti);
     // ---- end marks and the last partial bytes of every bitstream ----
 #pragma unroll
     for (int g = 0; g < G; g++) {
-      if (S.item[g].type == 1 && S.item[g].size > 1) {
+      if (kind[g] == 1) {
         uint32_t* bitbuf = S.bitbuf[warp][g];
         if (lane == 0) bitbuf[(st[g].B - 32 * st[g].flushed) >> 5] |= 1u << (st[g].B & 31);
         __syncwarp();

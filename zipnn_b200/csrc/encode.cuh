@@ -50,11 +50,13 @@ __device__ __forceinline__ uint32_t rot_byte_at(const uint8_t* __restrict__ in_c
 // pass A1: histograms.  Pure streaming: every input byte is read once (128-bit loads, four in
 // flight per thread), rotated, and counted with one shared-memory atomic.
 //
-// Counter layout rep[g][bin][col], col = lane % R, 32-bit counters: a warp's 32 atomics go to
+// Counter layout rep[bin][g][col], col = lane % R, 32-bit counters: a warp's 32 atomics go to
 // 32 / (32/R) distinct columns, so two lanes can only collide when they hold the same byte
-// value -- and the address is one shift + one LOP3 from the loaded word (3 instructions per
-// byte including the atomic; the first version spent 11).  Per stream quarter the columns are
-// folded into hist[item][stream][256] (u16) in global memory for pass A2.
+// value.  For G = 2 and 4 a bin's row is 256 bytes, so the counter's byte offset bin << 8 |
+// (g * R + col) * 4 is ONE PRMT of the loaded word with a per-lane, per-plane register: two
+// instructions per byte with the atomic.  G = 1 (128-byte rows) forms it with one multiply-add,
+// which keeps its footprint at 32 KiB.  Per pair of stream quarters the columns are folded
+// into hist[item][stream][256] (u16) in global memory for pass A2.
 // =====================================================================================
 // Columns per bin.  32 = one per lane: no two lanes of a warp ever meet in a bank (1 wavefront per
 // atomic instead of 2), at 32 KiB of counters per plane; fp32 has four planes and keeps 16.
@@ -62,13 +64,13 @@ __device__ __forceinline__ uint32_t rot_byte_at(const uint8_t* __restrict__ in_c
 template <int G>
 struct HistCfg {
   static constexpr int R = (G == 4) ? 16 : 32;
-  static constexpr int kShift = (G == 4) ? 6 : 7;      // log2(R * 4): byte offset of a bin
 };
 
 template <int G>
 struct HistSmem {
-  uint32_t rep[G][256][HistCfg<G>::R];
+  uint32_t rep[256][G][HistCfg<G>::R];
 };
+static_assert(sizeof(HistSmem<2>) == 256 * 256 && sizeof(HistSmem<4>) == 256 * 256, "PRMT address form needs 256-byte bin rows");
 
 template <int G>
 __global__ void __launch_bounds__(kEncThreads) k_encode_hist(const uint8_t* __restrict__ in, uint64_t n, uint32_t chunk,
@@ -77,15 +79,20 @@ __global__ void __launch_bounds__(kEncThreads) k_encode_hist(const uint8_t* __re
   HistSmem<G>& S = *reinterpret_cast<HistSmem<G>*>(smem_raw);
   constexpr int R = HistCfg<G>::R;
   const int tid = threadIdx.x, lane = tid & 31;
-  const uint32_t col_bytes = (uint32_t)(lane % R) * 4;
-  unsigned char* const col_p = reinterpret_cast<unsigned char*>(&S.rep[0][0][0]) + col_bytes;  // rep[0][0][lane % R]
-  for (int i = tid; i < G * 256 * R; i += kEncThreads) (&S.rep[0][0][0])[i] = 0;
+  unsigned char* const rep_b = reinterpret_cast<unsigned char*>(&S.rep[0][0][0]);
+  // byte offset of this lane's column of plane g within a bin row (< 256)
+  uint32_t col_b[G];
+#pragma unroll
+  for (int g = 0; g < G; g++) col_b[g] = (uint32_t)(g * R + lane % R) * 4;
+  for (int i = tid; i < 256 * G * R; i += kEncThreads) (&S.rep[0][0][0])[i] = 0;
   __syncthreads();
   for (uint64_t c = blockIdx.x; c < K; c += gridDim.x) {
     const uint8_t* in_c = in + c * (uint64_t)chunk;
     const uint32_t chunk_len = (c == K - 1) ? (uint32_t)(n - c * (uint64_t)chunk) : chunk;
     const uint32_t rot_words = (bits_mode == 1 && G > 1) ? (chunk_len >> 2) : 0;
     const bool fast = (chunk_len % 64u) == 0;
+    const uint32_t sign_m = rot_words ? ((G == 2) ? 0x00800080u : 0x00800000u) : 0u;  // where the sign bits go
+    const uint32_t exp_sh = rot_words ? 1u : 0u;
     for (int q = 0; q < 4; q++) {
       // Two stream quarters share one fold: quarter q counts in the low (q even) or high (q odd) half
       // of the 32-bit counters.  A column receives at most 8 threads x 128 bytes = 1024 per quarter,
@@ -116,15 +123,25 @@ __global__ void __launch_bounds__(kEncThreads) k_encode_hist(const uint8_t* __re
               uint32_t w[4] = {v[k].x, v[k].y, v[k].z, v[k].w};
 #pragma unroll
               for (int i = 0; i < 4; i++) {
-                if (rot_words) w[i] = rot_word<G>(w[i]);
+                // The sign-bit rotation (rot_word) never builds the rotated word: the exponent bytes are
+                // bytes of w << 1, and the sign | mantissa bytes are bytes of one bit-select of w and w >> 8
+                // (3 instructions per word instead of 5).
+                // Branch-free: without the rotation sign_m = 0 and exp_sh = 0 leave both equal to w.
+                uint32_t lo_w, hi_w = w[i] << exp_sh;
+                asm("lop3.b32 %0, %1, %2, %3, 0xD8;" : "=r"(lo_w) : "r"(w[i]), "r"(w[i] >> 8), "r"(sign_m));  // sign_m ? b : a
 #pragma unroll
                 for (int b = 0; b < 4; b++) {
-                  // byte b of the word -> address of its counter in THREE instructions: extract (PRMT with zeros),
-                  // bin * (R * 4) + this lane's column (one multiply-add on the FMA pipe), shared-memory reduction
-                  // with the plane as an immediate offset.  (Shift, mask | column, add the array base, ATOMS took four,
-                  // and the kernel is bound by instruction issue: profiles/r2p_encode_16GiB.summary.txt)
-                  const uint32_t byte = __byte_perm(w[i], 0u, 0x4440u | (uint32_t)b);
-                  atomicAdd(reinterpret_cast<uint32_t*>(col_p + ((4 * i + b) % G) * (256 * R * 4) + byte * (uint32_t)(R * 4)), inc);
+                  const uint32_t g = (4 * i + b) % G;
+                  const bool exp_byte = (G == 2 && (b & 1)) || (G == 4 && b == 3);
+                  uint32_t off;
+                  if constexpr (G == 1) {
+                    // extract (PRMT with zeros), then bin * 128 + column on the FMA pipe
+                    off = __byte_perm(w[i], 0u, 0x4440u | (uint32_t)b) * (uint32_t)(R * 4) + col_b[0];
+                  } else {
+                    // bytes (column, byte b, 0, 0): the counter's offset bin << 8 | column in one PRMT
+                    off = __byte_perm(exp_byte ? hi_w : lo_w, col_b[g], 0x6504u | ((uint32_t)b << 4));
+                  }
+                  atomicAdd(reinterpret_cast<uint32_t*>(rep_b + off), inc);
                 }
               }
             }
@@ -136,19 +153,24 @@ __global__ void __launch_bounds__(kEncThreads) k_encode_hist(const uint8_t* __re
           const uint32_t seg = (pl + 3) >> 2;
           const uint32_t j0 = min(pl, (uint32_t)q * seg), j1 = (q == 3) ? pl : min(pl, j0 + seg);
           for (uint32_t j = j0 + tid; j < j1; j += kEncThreads)
-            atomicAdd(&S.rep[g][rot_byte_at<G>(in_c, chunk_len, rot_words, j * G + g)][lane % R], inc);
+            atomicAdd(&S.rep[rot_byte_at<G>(in_c, chunk_len, rot_words, j * G + g)][g][lane % R], inc);
         }
       }
       if ((q & 1) == 0) continue;
       __syncthreads();
-      // fold the columns of each bin (and clear them); thread t owns bin t of every group
-      for (int g = 0; g < G; g++) {
+      // fold the columns of each bin (and clear them); thread t owns bin t of every group.  128-bit
+      // accesses, rotated by thread so the eight lanes of an access phase hit distinct banks (G = 4:
+      // lanes 4..7 of each phase take the neighbouring plane for the same reason).
+      for (int g0 = 0; g0 < G; g0++) {
+        const int g = (G == 4) ? (g0 ^ ((tid >> 2) & 1)) : g0;
+        uint4* row = reinterpret_cast<uint4*>(&S.rep[tid][g][0]);
         uint32_t sum = 0;
 #pragma unroll
-        for (int r = 0; r < R; r++) {
-          const int rr = (r + tid) % R;
-          sum += S.rep[g][tid][rr];
-          S.rep[g][tid][rr] = 0;
+        for (int r = 0; r < R / 4; r++) {
+          const int rr = (r + tid) % (R / 4);
+          const uint4 x = row[rr];
+          sum += x.x + x.y + x.z + x.w;
+          row[rr] = make_uint4(0, 0, 0, 0);
         }
         uint16_t* h = hist + (((uint64_t)g * K + c) * 4 + (q - 1)) * 256 + tid;
         h[0] = (uint16_t)(sum & 0xFFFFu);
@@ -172,6 +194,210 @@ struct __align__(16) TableWarp {
   TreeScratch tree;
 };
 constexpr int kTableWarps = 4;
+
+// tANS bytes of the weights T.weight[0..n) (huf_pack_weights' encoder, lines after fse_write_ncount), one warp.
+// E.norm holds the normalised counts of the weights 0..max_w at table log lgf (5 or 6).  The spread, the
+// next-state table and the per-symbol deltas are built by lane (fse_build_enc), the two interleaved state
+// chains run on lane 0 over per-position deltas prepared by lane, and the emitted bits are placed by a warp
+// prefix sum.  Scratch: T.cnt (per-position deltas), T.parent (emissions), T.depth (bit words).  Returns the
+// byte count written to dst; every lane gets it.
+__device__ int warp_fse_encode(TreeScratch& T, int n, int max_w, int lgf, uint8_t* dst) {
+  const int lane = threadIdx.x & 31;
+  const unsigned full = 0xffffffffu, lt = (1u << lane) - 1u;
+  FseEnc& E = T.fse;
+  const uint32_t size = 1u << lgf, mask = size - 1, step = (size >> 1) + (size >> 3) + 3;
+  // ---- per symbol (lane s <= max_w <= 12): cumul, place of the low-probability symbols, deltas
+  const bool is_sym = lane <= max_w;
+  const int nrm = is_sym ? E.norm[lane] : 0;
+  const uint32_t slots = nrm == -1 ? 1u : (nrm > 0 ? (uint32_t)nrm : 0u);  // cumul increment
+  const uint32_t occ = nrm > 0 ? (uint32_t)nrm : 0u;                      // slots taken by the spread walk
+  uint32_t cum = slots, pstart = occ;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t a = __shfl_up_sync(full, cum, o), b = __shfl_up_sync(full, pstart, o);
+    if (lane >= o) { cum += a; pstart += b; }
+  }
+  cum -= slots;
+  pstart -= occ;
+  const uint32_t low = __ballot_sync(full, is_sym && nrm == -1);
+  const uint32_t high = size - 1 - __popc(low);
+  if (is_sym && nrm == -1) E.spread[size - 1 - __popc(low & lt)] = (uint8_t)lane;
+  uint32_t db = 0;
+  int32_t df = 0;
+  if (nrm == 0) {
+    db = ((uint32_t)(lgf + 1) << 16) - size;
+  } else if (nrm == -1 || nrm == 1) {
+    db = ((uint32_t)lgf << 16) - size;
+    df = (int32_t)cum - 1;
+  } else {
+    const uint32_t max_out = (uint32_t)lgf - (uint32_t)hb32((uint32_t)(nrm - 1));
+    db = (max_out << 16) - ((uint32_t)nrm << max_out);
+    df = (int32_t)cum - nrm;
+  }
+  // ---- spread: the positions j * step & mask (j = 0, 1, ..) that are <= high take the positive symbols'
+  // slots in symbol order, which is the walk of fse_build_enc with its skips
+  uint32_t before = 0;
+  for (uint32_t j0 = 0; j0 < size; j0 += 32) {
+    const uint32_t u = ((j0 + lane) * step) & mask;
+    const bool valid = u <= high;
+    const uint32_t vm = __ballot_sync(full, valid);
+    const uint32_t r = before + __popc(vm & lt);
+    before += __popc(vm);
+    int sym = 0;
+    for (int s = 0; s <= max_w; s++) {
+      const uint32_t ps = __shfl_sync(full, pstart, s), pc = __shfl_sync(full, occ, s);
+      if (r >= ps && r < ps + pc) sym = s;
+    }
+    if (valid) E.spread[u] = (uint8_t)sym;
+  }
+  if (is_sym) E.cumul[lane] = cum;
+  if (lane < 16) E.count[lane] = 0;  // reused: occurrences of each symbol in spread[0, 32)
+  __syncwarp();
+  // ---- next_state[cumul[s] + k] = size + u for the k-th u with spread[u] = s
+  {
+    const uint32_t s0 = E.spread[lane];
+    const uint32_t m0 = __match_any_sync(full, s0);
+    E.next_state[E.cumul[s0] + __popc(m0 & lt)] = (uint16_t)(size + lane);
+    if (size > 32) {
+      E.count[s0] = __popc(m0);
+      __syncwarp();
+      const uint32_t s1 = E.spread[32 + lane];
+      const uint32_t m1 = __match_any_sync(full, s1);
+      E.next_state[E.cumul[s1] + E.count[s1] + __popc(m1 & lt)] = (uint16_t)(size + 32 + lane);
+    }
+  }
+  // ---- the deltas of the weight at every position
+  uint32_t* pdb = T.cnt;
+  int32_t* pdf = reinterpret_cast<int32_t*>(T.cnt + 256);
+  for (int i0 = 0; i0 < n; i0 += 32) {
+    const int i = i0 + lane;
+    const int w = i < n ? T.weight[i] : 0;
+    const uint32_t a = __shfl_sync(full, db, w);
+    const int32_t b = __shfl_sync(full, df, w);
+    if (i < n) {
+      pdb[i] = a;
+      pdf[i] = b;
+    }
+  }
+  __syncwarp();
+  // ---- the two state chains (huf_pack_weights' order): emissions value | nbits << 8
+  uint16_t* em = T.parent;
+  int nem = 0;
+  if (lane == 0) {
+    const uint16_t* ns = E.next_state;
+    auto seed = [&](int i) {
+      const uint32_t d = pdb[i], nb = (d + (1u << 15)) >> 16;
+      return (uint32_t)ns[(int32_t)((((nb << 16) - d)) >> nb) + pdf[i]];
+    };
+    auto emit = [&](uint32_t st, int i) {
+      const uint32_t nb = (st + pdb[i]) >> 16;
+      em[nem++] = (uint16_t)((st & ((1u << nb) - 1u)) | (nb << 8));
+      return (uint32_t)ns[(int32_t)(st >> nb) + pdf[i]];
+    };
+    int ip = n;
+    uint32_t s1, s2;
+    if (n & 1) {
+      s1 = seed(--ip);
+      s2 = seed(--ip);
+      s1 = emit(s1, --ip);
+    } else {
+      s2 = seed(--ip);
+      s1 = seed(--ip);
+    }
+    while (ip > 0) {
+      s2 = emit(s2, --ip);
+      s1 = emit(s1, --ip);
+    }
+    em[nem++] = (uint16_t)((s2 & mask) | ((uint32_t)lgf << 8));
+    em[nem++] = (uint16_t)((s1 & mask) | ((uint32_t)lgf << 8));
+    em[nem++] = (uint16_t)(1u | (1u << 8));  // end mark
+  }
+  nem = __shfl_sync(full, nem, 0);
+  // ---- place the emissions LSB first: warp prefix sum of their lengths, OR into words
+  uint32_t* words = reinterpret_cast<uint32_t*>(T.depth);
+  for (int i = lane; i < 128; i += 32) words[i] = 0;
+  __syncwarp();
+  uint32_t at = 0;
+  for (int e0 = 0; e0 < nem; e0 += 32) {
+    const uint32_t v = (e0 + lane < nem) ? em[e0 + lane] : 0u;
+    const uint32_t len = v >> 8;
+    uint32_t x = len;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t y = __shfl_up_sync(full, x, o);
+      if (lane >= o) x += y;
+    }
+    const uint32_t off = at + x - len, bits = v & 0xFFu;
+    if (len) {
+      atomicOr(&words[off >> 5], bits << (off & 31));
+      if ((off & 31) + len > 32) atomicOr(&words[(off >> 5) + 1], bits >> (32 - (off & 31)));
+    }
+    at += __shfl_sync(full, x, 31);
+  }
+  __syncwarp();
+  const int bytes = (int)((at + 7) >> 3);
+  for (int i = lane; i < bytes; i += 32) dst[i] = (uint8_t)(words[i >> 2] >> (8 * (i & 3)));
+  __syncwarp();
+  return bytes;
+}
+
+// Table description from the code lengths nb[256], one warp: the bytes of huf_write_table (huf_serial.cuh,
+// which the host tests fuzz against the oracle), with the weights, their histogram, the tANS tables and
+// the nibble form built by lane.  Writes T.hdr; returns its size or -1 (block kept raw), on every lane.
+__device__ int warp_write_table(TreeScratch& T, const uint8_t* nb, int max_sym, int lg) {
+  const int lane = threadIdx.x & 31;
+  const unsigned full = 0xffffffffu;
+  FseEnc& E = T.fse;
+  const int n = max_sym;  // weights of symbols 0..max_sym-1 are sent, the last one is implied
+  if (lane < 16) E.count[lane] = 0;
+  __syncwarp();
+  int max_w = 0;
+  for (int s = lane; s <= n; s += 32) {
+    const uint32_t w = (s < n && nb[s]) ? (uint32_t)(lg + 1 - nb[s]) : 0u;
+    T.weight[s] = (uint8_t)w;  // weight[max_sym] = 0 pads the nibble form
+    if (s < n) {
+      atomicAdd(&E.count[w], 1u);
+      max_w = max(max_w, (int)w);
+    }
+  }
+  max_w = __reduce_max_sync(full, max_w);
+  __syncwarp();
+  // ---- huf_pack_weights' decisions; h = its return value
+  int h = 0;
+  if (n > 1) {
+    const uint32_t top = __reduce_max_sync(full, lane <= max_w ? E.count[lane] : 0u);
+    if (top == (uint32_t)n) {
+      h = 1;
+    } else if (top > 1) {
+      const int lgf = fse_pick_log(6, (uint32_t)n, (uint32_t)max_w, 2);
+      int hn = -1;
+      if (lane == 0 && fse_normalize(E.norm, lgf, E.count, (uint32_t)n, max_w) == 0)
+        hn = fse_write_ncount(T.hdr + 1, E.norm, max_w, lgf);
+      hn = __shfl_sync(full, hn, 0);
+      __syncwarp();
+      if (hn < 0) {
+        h = -1;
+      } else if (n <= 2) {
+        h = 0;
+      } else if (hn + 1 >= max_sym / 2) {
+        h = hn + 1;  // the bitstream adds at least one byte, so the nibble form (or raw) is chosen anyway
+      } else {
+        h = hn + warp_fse_encode(T, n, max_w, lgf, T.hdr + 1 + hn);
+      }
+    }
+  }
+  if (h < 0) return -1;
+  if (h > 1 && h < max_sym / 2) {
+    if (lane == 0) T.hdr[0] = (uint8_t)h;
+    __syncwarp();
+    return h + 1;
+  }
+  if (max_sym > 128) return -1;
+  if (lane == 0) T.hdr[0] = (uint8_t)(128 + (max_sym - 1));
+  for (int s = 2 * lane; s < max_sym; s += 64) T.hdr[(s / 2) + 1] = (uint8_t)((T.weight[s] << 4) + T.weight[s + 1]);
+  __syncwarp();
+  return ((max_sym + 1) / 2) + 1;
+}
 
 // hist = this item's four per-stream histograms, u16[4][256] in global memory (read twice: totals, exact sizes)
 __device__ void warp_block_decision(TableWarp& S, const uint16_t* __restrict__ hist, uint32_t plen, double thr, uint8_t* type_out,
@@ -235,15 +461,14 @@ __device__ void warp_block_decision(TableWarp& S, const uint16_t* __restrict__ h
       T.sym[rank] = nz[i];
     }
     __syncwarp();
-    int lg = 0, hsize = -1;
-    if (lane == 0) {
-      const int want = fse_pick_log(kHufLogDefault, plen, (uint32_t)max_sym, 1);
-      lg = huf_lengths_from_sorted(T, k - 1, want, S.nb);
-      hsize = huf_write_table(T, S.nb, max_sym, lg);
-    }
+    int lg = 0;
+    if (lane == 0) lg = huf_tree_depths(T, k - 1, fse_pick_log(kHufLogDefault, plen, (uint32_t)max_sym, 1));
+    for (int s = lane; s < 256; s += 32) S.nb[s] = 0;
     lg = __shfl_sync(0xffffffffu, lg, 0);
-    hsize = __shfl_sync(0xffffffffu, hsize, 0);
     __syncwarp();
+    for (int i = lane; i < k; i += 32) S.nb[T.sym[i]] = T.depth[i];
+    __syncwarp();
+    const int hsize = warp_write_table(T, S.nb, max_sym, lg);
     if (hsize > 0 && (uint32_t)hsize + 12 < plen && plen >= 12) {
       uint32_t bits[4] = {0, 0, 0, 0};
       for (int s = lane; s <= max_sym; s += 32) {

@@ -442,9 +442,9 @@ ZB_HD inline int huf_limit_depth(TreeScratch& T, int last, int max_nb) {
 }
 
 // Input: T.cnt[0..last], T.sym[0..last] = the symbols with non-zero count ordered by
-// (count descending, symbol ascending); last >= 1.  Output: nb_out[256] by symbol.
-// Returns the table log (largest code length).
-ZB_HD inline int huf_lengths_from_sorted(TreeScratch& T, int last, int max_nb, uint8_t* nb_out) {
+// (count descending, symbol ascending); last >= 1.  Output: T.depth[0..last], the code length
+// of sorted leaf n.  Returns the table log (largest code length).
+ZB_HD inline int huf_tree_depths(TreeScratch& T, int last, int max_nb) {
   const int kFirst = 256;
   const uint32_t kWall = 0x80000000u;
   int low_leaf = last, low_int = kFirst, next = kFirst;
@@ -466,7 +466,12 @@ ZB_HD inline int huf_lengths_from_sorted(TreeScratch& T, int last, int max_nb, u
   T.depth[root] = 0;
   for (int n = root - 1; n >= kFirst; n--) T.depth[n] = (uint8_t)(T.depth[T.parent[n]] + 1);
   for (int n = 0; n <= last; n++) T.depth[n] = (uint8_t)(T.depth[T.parent[n]] + 1);
-  const int lg = huf_limit_depth(T, last, max_nb);
+  return huf_limit_depth(T, last, max_nb);
+}
+
+// huf_tree_depths, then nb_out[256] by symbol.
+ZB_HD inline int huf_lengths_from_sorted(TreeScratch& T, int last, int max_nb, uint8_t* nb_out) {
+  const int lg = huf_tree_depths(T, last, max_nb);
   for (int s = 0; s < 256; s++) nb_out[s] = 0;
   for (int n = 0; n <= last; n++) nb_out[T.sym[n]] = T.depth[n];
   return lg;
@@ -508,6 +513,7 @@ ZB_HD inline void huf_assign_values(const uint8_t* nb, int max_sym, int lg, uint
 
 // Table description.  Writes into T.hdr; returns its size, or -1 when the block must
 // be stored raw (alphabet too large for the nibble form and tANS did not pay off).
+// The encode kernel writes the same bytes with a whole warp (warp_write_table, encode.cuh).
 ZB_HD inline int huf_write_table(TreeScratch& T, const uint8_t* nb, int max_sym, int lg) {
   for (int s = 0; s < max_sym; s++) T.weight[s] = nb[s] ? (uint8_t)(lg + 1 - nb[s]) : 0;
   int h = huf_pack_weights(T.hdr + 1, T.weight, max_sym, T.fse);
